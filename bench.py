@@ -7,6 +7,7 @@ and the reference's CPU path timed on the same box.
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU path (pandas restatement)
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's result as DIR/grp.npy, DIR/rev.npy
 
 Headline workload (SURVEY 8d, seed 4): fact(fk int64, x int64, val float64) with --rows rows in
 total (default 1e9, strong scaling: rows/N per GPU, 8 partitions spread over the GPUs),
@@ -72,7 +73,15 @@ def parse_args():
                     help="comma list of C1,C2,C2i,C2z,C3,C3f,C4s,C5 (default all)")
     ap.add_argument("--config-scale", type=float, default=float(os.environ.get("B200SQL_CONFIG_SCALE", 1.0)),
                     help="scale the row counts of the extra configs (smoke runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result of the last one as DIR/<column>.npy (float64, "
+                         "rows ordered by the group key), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's result; it does not apply to --impl reference")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -327,6 +336,9 @@ def main():
     free_b, total_b = torch.cuda.mem_get_info()
     need = n_local * BYTES_PER_FACT_ROW * 1.15 + DIM_ROWS * 24 * 4
     if need > free_b:
+        if args.dump_outputs:   # the inputs, and so the dumped result, would depend on the free memory
+            raise SystemExit(f"[bench] {n_total} fact rows do not fit this GPU's free HBM; pass a smaller --rows "
+                             "to --dump-outputs")
         n_local = int((free_b - DIM_ROWS * 96) / (BYTES_PER_FACT_ROW * 1.15))
         n_total = n_local * world
         print(f"[bench] shrinking to {n_total} fact rows to fit HBM", file=sys.stderr)
@@ -432,6 +444,8 @@ def main():
     if sampler.is_alive():
         sampler.join(timeout=2)
     n_groups_local = parts[0].n
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, parts, rank)
 
     peak_gbs, peak_src = load_peaks()
     traffic = load_traffic()
@@ -555,6 +569,34 @@ def verify_full_size(torch, dist, world, parts, fk, x, val, pk, flag, grp):
             "groups_expected": groups_expected, "keys_unique": bool(unique and disjoint),
             "rows_contributing": int(rows.item()), "ranks": world,
             "ok": bool(rel <= 1e-9 and groups == groups_expected and unique and disjoint)}
+
+
+RESULT_COLUMNS = ("grp", "rev")      # QUERY's output columns, group key first
+DUMP_ARRAY_BYTES = 63 * 10**6        # the .npy files stay under 64 MB in all, headers included
+
+
+def dump_outputs(out_dir, parts, rank):
+    """Write the result of the timed query, the columns a caller of Context.sql(QUERY) receives, as
+    out_dir/<column>.npy in float64 (the int64 group keys are far below 2**53, so exactly).  SQL leaves
+    the order of GROUP BY output open and two builds may emit it differently, so rows are ordered by the
+    group key.  A result larger than DUMP_ARRAY_BYTES is written as a fixed, seeded sample of its rows.
+    N>1: the ranks' key ranges are gathered (a collective, every rank calls it) and rank 0 writes."""
+    import numpy as np
+    import pandas as pd
+    from dask_sql_b200 import device as D, executor
+    parts = [executor.gather_keyrange(p) for p in parts]
+    if rank != 0:
+        return
+    frame = pd.concat([pd.DataFrame({c: D.column_to_host(p[c]) for c in RESULT_COLUMNS}) for p in parts],
+                      ignore_index=True)
+    cols = {c: frame[c].to_numpy(dtype=np.float64, na_value=np.nan) for c in RESULT_COLUMNS}
+    order = np.argsort(cols[RESULT_COLUMNS[0]], kind="stable")
+    keep = DUMP_ARRAY_BYTES // (8 * len(cols))
+    if len(order) > keep:
+        order = order[np.sort(np.random.default_rng(0).choice(len(order), keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for c, v in cols.items():
+        np.save(os.path.join(out_dir, c + ".npy"), v[order])
 
 
 def run_e2e(args, torch, dist, dev, world, rank, fk, x, val, pk, flag, grp, fact_dist, dim_dist, barrier,
