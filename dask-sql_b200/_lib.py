@@ -92,6 +92,23 @@ class PeerMerge(C.Structure):
                 ("epoch", C.c_uint64)]
 
 
+WIN_MAX_KEYS = 8
+WB_UNBOUNDED, WB_OFFSET = 0, 1
+(WIN_ROW_NUMBER, WIN_RANK, WIN_DENSE_RANK, WIN_SUM, WIN_COUNT, WIN_AVG, WIN_MIN, WIN_MAX, WIN_FIRST,
+ WIN_LAST) = range(10)
+
+
+class WSegs(C.Structure):
+    _fields_ = [("part_start", C.c_void_p), ("part_end", C.c_void_p), ("peer_start", C.c_void_p),
+                ("peer_end", C.c_void_p), ("dense", C.c_void_p)]
+
+
+class WFrame(C.Structure):
+    _fields_ = [("range", C.c_int32), ("lo_kind", C.c_int32), ("hi_kind", C.c_int32), ("pad_", C.c_int32),
+                ("lo", C.c_int64), ("hi", C.c_int64)]
+
+
+assert C.sizeof(WSegs) == 40 and C.sizeof(WFrame) == 32
 assert C.sizeof(Col) == 24 and C.sizeof(Term) == 32 and C.sizeof(Scan) == 656
 assert C.sizeof(AggState) == 152 and C.sizeof(Instr) == 24 and C.sizeof(Prog) == 1544
 assert C.sizeof(JoinTable) == 152 and C.sizeof(StarLookup) == 56 and C.sizeof(PeerMerge) == 544
@@ -188,10 +205,15 @@ _SIGS = {
     "b2_star_build_hash": [C.POINTER(Col), _P, C.c_int64, _P, _P, _P, C.c_int64, _P, _P],
     "b2_star_agg": [C.POINTER(Scan), C.c_int32, C.POINTER(StarLookup), C.POINTER(Agg), C.c_int32,
                     C.POINTER(AggState), _P],
+    "b2_window_segments": [C.POINTER(Col), C.c_int32, C.c_int32, C.c_int64, C.POINTER(WSegs), _P, _P],
+    "b2_window_rank": [C.c_int32, C.c_int64, C.POINTER(WSegs), _P, _P],
+    "b2_window_offset": [C.POINTER(Col), C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.POINTER(WSegs), _P, _P, _P],
+    "b2_window_agg": [C.POINTER(Col), C.c_int32, C.POINTER(WFrame), C.c_int64, C.POINTER(WSegs), _P, _P, _P, _P],
 }
 
 EXPORTS = sorted(list(_SIGS) + ["b2_last_error", "b2_num_tiles", "b2_stats_ws_bytes", "b2_scan_agg_ws_bytes",
-                                "b2_sort_ws_bytes", "b2_join_onepass_ws_bytes", "b2_range_partition_ws_bytes",
+                                "b2_sort_ws_bytes", "b2_window_ws_bytes", "b2_join_onepass_ws_bytes",
+                                "b2_range_partition_ws_bytes",
                                 "b2_f64_to_ordered", "b2_ordered_to_f64"])
 
 
@@ -275,6 +297,13 @@ star_build_dense = _wrap("b2_star_build_dense")
 star_build_scan = _wrap("b2_star_build_scan")
 star_build_hash = _wrap("b2_star_build_hash")
 star_agg = _wrap("b2_star_agg")
+window_segments = _wrap("b2_window_segments")
+window_rank = _wrap("b2_window_rank")
+window_offset = _wrap("b2_window_offset")
+window_agg = _wrap("b2_window_agg")
+_lib.b2_window_ws_bytes.restype = C.c_int64
+_lib.b2_window_ws_bytes.argtypes = [C.c_int64]
+window_ws_bytes = _lib.b2_window_ws_bytes
 num_tiles = _lib.b2_num_tiles
 stats_ws_bytes = _lib.b2_stats_ws_bytes
 scan_agg_ws_bytes = _lib.b2_scan_agg_ws_bytes

@@ -39,6 +39,7 @@ int b2_sm_count() {
 #include "sort.cuh"
 #include "partition.cuh"
 #include "peer.cuh"
+#include "window.cuh"
 
 extern "C" {
 

@@ -89,7 +89,16 @@ __device__ __forceinline__ uint64_t b2_ld_volatile_u64(const uint64_t* p) {
 __device__ __forceinline__ void b2_st_volatile_u64(uint64_t* p, uint64_t v) {
   asm volatile("st.volatile.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
-__device__ __forceinline__ int64_t b2_lookback(uint64_t* __restrict__ status, int64_t tile, int64_t agg, int lane) {
+// The combining operator is a template parameter: commutative and associative over non-negative
+// values below 2^62, with identity 0 (sum of counts; max of row positions, window.cuh).
+struct b2_lb_sum {
+  static __device__ __forceinline__ int64_t op(int64_t a, int64_t b) { return a + b; }
+};
+struct b2_lb_max {
+  static __device__ __forceinline__ int64_t op(int64_t a, int64_t b) { return a > b ? a : b; }
+};
+template <class OP>
+__device__ __forceinline__ int64_t b2_lookback_op(uint64_t* __restrict__ status, int64_t tile, int64_t agg, int lane) {
   if (tile == 0) {
     if (lane == 0) b2_st_volatile_u64(status, B2_LB_PREFIX | (uint64_t)agg);
     return 0;
@@ -106,12 +115,15 @@ __device__ __forceinline__ int64_t b2_lookback(uint64_t* __restrict__ status, in
     const int first = pmask ? __ffs(pmask) - 1 : 31;    // nearest lane holding an inclusive prefix
     int64_t val = lane <= first ? (int64_t)(v & B2_LB_MASK) : 0;
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) val += __shfl_xor_sync(FULL_MASK, val, o);
-    excl += val;
+    for (int o = 16; o > 0; o >>= 1) val = OP::op(val, __shfl_xor_sync(FULL_MASK, val, o));
+    excl = OP::op(excl, val);
     if (pmask) break;
   }
-  if (lane == 0) b2_st_volatile_u64(status + tile, B2_LB_PREFIX | (uint64_t)(excl + agg));
+  if (lane == 0) b2_st_volatile_u64(status + tile, B2_LB_PREFIX | (uint64_t)OP::op(excl, agg));
   return excl;
+}
+__device__ __forceinline__ int64_t b2_lookback(uint64_t* __restrict__ status, int64_t tile, int64_t agg, int lane) {
+  return b2_lookback_op<b2_lb_sum>(status, tile, agg, lane);
 }
 
 __device__ __forceinline__ bool b2_bit(const uint8_t* __restrict__ bm, int64_t i) {

@@ -25,7 +25,7 @@ from . import expr as E
 from . import parallel as P
 from .device import DeviceColumn, TermSpec, I64, F64, U8
 from .expr import Expr, ColRef, Lit, Call
-from .frame import LazyFrame, Source, TableSource, JoinSource, AggSource, SortSource, LimitSource
+from .frame import LazyFrame, Source, TableSource, JoinSource, AggSource, SortSource, LimitSource, WindowSource
 from .table import DeviceTable, HostColumn
 
 DENSE_MAX_SLOTS = 1 << 27          # direct-address group tables up to 128M slots
@@ -426,7 +426,7 @@ def frame_distribution(frame: LazyFrame) -> str:
         return src.table.distribution
     if isinstance(src, JoinSource):
         return join_sides(src)[1]
-    if isinstance(src, (SortSource, LimitSource)):
+    if isinstance(src, (SortSource, LimitSource, WindowSource)):
         return "replicated" if P.world()[1] > 1 else "local"
     return "replicated" if P.world()[1] > 1 else "local"
 
@@ -542,6 +542,8 @@ def materialize(src: Source, needed: Set[str], top: bool = False, pred=None) -> 
         return [run_sort(src, needed)]
     if isinstance(src, LimitSource):
         return [run_limit(src, needed)]
+    if isinstance(src, WindowSource):
+        return [run_window(src, needed)]
     raise TypeError(f"unknown source {type(src).__name__}")
 
 
@@ -567,6 +569,137 @@ def run_sort(src: SortSource, needed: Set[str]) -> Part:
             stats["launches"] += 1
             out[k] = D.gather(whole[k], idx, False)
     return out
+
+
+_WIN_OP = {"row_number": L.WIN_ROW_NUMBER, "rank": L.WIN_RANK, "dense_rank": L.WIN_DENSE_RANK, "sum": L.WIN_SUM,
+           "count": L.WIN_COUNT, "avg": L.WIN_AVG, "min": L.WIN_MIN, "max": L.WIN_MAX, "first_value": L.WIN_FIRST,
+           "last_value": L.WIN_LAST}
+
+
+def run_window(src: WindowSource, needed: Set[str]) -> Part:
+    """Window functions (window.py:227-348 of the reference: one groupby().apply() per call).  The child
+    is made whole (and, at world > 1, gathered from its shards: every rank computes the same rows);
+    calls with identical (PARTITION BY, ORDER BY) share one sort -- b2_sort_by per key, order keys then
+    partition keys, last key first -- and one gather of the columns still needed, then
+    b2_window_segments and one kernel per call.  The result is in the last sort's row order."""
+    dev = _dev()
+    refs = set()
+    for w in src.calls:
+        refs.update(w.args)
+        refs.update(w.partition)
+        refs.update(k for k, _, _ in w.order)
+    names = [n for n in src.child.columns if n in needed or n in refs]
+    whole = concat_parts(execute(src.child, names), names)
+    if P.world()[1] > 1 and frame_distribution(src.child) in ("sharded", "root"):
+        from .merge import allgather_part
+        with _Phase("window_gather"):
+            whole = allgather_part(Part(dict(whole), whole.n), dev)
+    n = whole.n
+    if n >= 1 << 31:
+        raise NotImplementedError(f"window functions over {n} rows: the input must hold fewer than 2^31 rows "
+                                  "(the sort's int32 row ids)")
+    calls = [w for w in src.calls if w.out in needed]
+    specs: Dict[tuple, list] = {}
+    for w in calls:
+        specs.setdefault((tuple(w.partition), tuple(w.order)), []).append(w)
+    cur = {k: whole[k] for k in names}
+    if n == 0:
+        for w in calls:
+            dt, lg = src.schema[w.out]
+            cur[w.out] = DeviceColumn(torch.empty(0, dtype=_TORCH_DT[dt], device=dev), None, dt, lg)
+        return Part({k: cur[k] for k in src.schema if k in needed}, 0)
+    ws = torch.empty(max(L.sort_ws_bytes(n), L.window_ws_bytes(n)), dtype=torch.uint8, device=dev)
+    seg = torch.empty((5, n), dtype=torch.int32, device=dev)
+    segs = L.WSegs(*[seg[i].data_ptr() for i in range(5)])
+    for (part_keys, order_keys), group in specs.items():
+        keys = [(k, True, False) for k in part_keys] + list(order_keys)
+        if len(keys) > L.WIN_MAX_KEYS:
+            raise NotImplementedError(f"a window partitions and orders by at most {L.WIN_MAX_KEYS} columns")
+        if keys:
+            idx = torch.empty(n, dtype=torch.int32, device=dev)
+            rec = _kernel_event_begin("window_sort", n)
+            stats["launches"] += 1
+            L.iota(D.ptr(idx), n, D.stream_ptr())
+            for name, asc, nulls_first in reversed(keys):
+                cs = cur[name].as_struct()
+                stats["launches"] += 29
+                L.sort_by(C.byref(cs), n, 0 if asc else 1, 1 if nulls_first else 0, D.ptr(idx), D.ptr(ws),
+                          D.stream_ptr())
+            _kernel_event_end(rec)
+            rec = _kernel_event_begin("window_gather", n)
+            for k in list(cur):
+                stats["launches"] += 1
+                cur[k] = D.gather(cur[k], idx, False)
+            _kernel_event_end(rec)
+        kc = (L.Col * max(1, len(keys)))(*[cur[k].as_struct() for k, _, _ in keys])
+        rec = _kernel_event_begin("window_segments", n)
+        stats["launches"] += 3
+        L.window_segments(kc, len(part_keys), len(keys), n, C.byref(segs), D.ptr(ws), D.stream_ptr())
+        _kernel_event_end(rec)
+        for w in group:
+            rec = _kernel_event_begin("window_" + w.func, n)
+            cur[w.out] = _window_call(w, cur, n, segs, ws, src.schema[w.out][1])
+            _kernel_event_end(rec)
+        stats["window_specs"] = stats.get("window_specs", 0) + 1
+    return Part({k: cur[k] for k in src.schema if k in needed}, n)
+
+
+def _frame_struct(frame) -> "L.WFrame":
+    unit, lo, hi = frame
+
+    def bound(b):
+        kind, off = b
+        if kind.startswith("UNBOUNDED"):
+            return L.WB_UNBOUNDED, 0
+        if kind == "CURRENT":
+            return L.WB_OFFSET, 0
+        return L.WB_OFFSET, (-off if kind == "PRECEDING" else off)
+
+    (lk, lo_off), (hk, hi_off) = bound(lo), bound(hi)
+    return L.WFrame(1 if unit == "RANGE" else 0, lk, hk, 0, lo_off, hi_off)
+
+
+def _window_call(w, cur, n, segs, ws, logical) -> DeviceColumn:
+    dev = _dev()
+    if w.func in ("row_number", "rank", "dense_rank"):
+        out = torch.empty(n, dtype=torch.int64, device=dev)
+        stats["launches"] += 1
+        L.window_rank(_WIN_OP[w.func], n, C.byref(segs), D.ptr(out), D.stream_ptr())
+        return DeviceColumn(out, None, I64)
+    val = cur[w.args[0]] if w.args else None
+    back_to_bool = False
+    if val is not None and val.dtype == U8:
+        # booleans run as int64 0/1 (SUM counts TRUEs); MIN / MAX / FIRST / LAST / LAG / LEAD cast back
+        stats["launches"] += 1
+        val = eval_expr(Part({"v": val}, n), E.cast(ColRef("v", U8), I64))
+        back_to_bool = w.func not in ("sum", "count", "avg")
+    vs = val.as_struct() if val is not None else L.Col()
+    valid = torch.empty(D.bitmap_words(n), dtype=torch.int32, device=dev)
+    if w.func in ("lag", "lead"):
+        k, default = w.params
+        out = torch.empty(n, dtype=_TORCH_DT[val.dtype], device=dev)
+        raw = 0
+        if default is not None:
+            raw = int(np.array([default], dtype=np.float64 if val.dtype == F64 else np.int64).view(np.int64)[0])
+        stats["launches"] += 1
+        L.window_offset(C.byref(vs), n, -k if w.func == "lag" else k, default is not None, raw, C.byref(segs),
+                        D.ptr(out), D.ptr(valid), D.stream_ptr())
+        dt = val.dtype
+    else:
+        dt = I64 if w.func == "count" else F64 if w.func == "avg" else val.dtype
+        out = torch.empty(n, dtype=_TORCH_DT[dt], device=dev)
+        if w.func == "count":
+            valid = None
+        fr = _frame_struct(w.frame)
+        stats["launches"] += 4
+        L.window_agg(C.byref(vs), _WIN_OP[w.func], C.byref(fr), n, C.byref(segs), D.ptr(out), D.ptr(valid),
+                     D.ptr(ws), D.stream_ptr())
+    res = DeviceColumn(out, valid, dt, logical if dt != U8 else None)
+    if back_to_bool:
+        stats["launches"] += 1
+        res = eval_expr(Part({"v": res}, n), E.cast(ColRef("v", I64), U8))
+        res.logical = logical
+    return res
 
 
 def run_limit(src: LimitSource, needed: Set[str]) -> Part:

@@ -14,7 +14,7 @@ so chains of Filter / Projection / TableScan nodes collapse into ONE fused kerne
 """
 import itertools
 from collections import OrderedDict
-from typing import Dict, List, Sequence
+from typing import Dict, List, NamedTuple, Sequence
 
 import numpy as np
 
@@ -90,6 +90,40 @@ class SortSource(Source):
     def __init__(self, child: "LazyFrame", keys):
         self.child, self.keys = child, list(keys)
         self.schema = OrderedDict((n, child.col_type(n)) for n in child.columns)
+
+
+class WindowCall(NamedTuple):
+    """One window function of a WindowSource.  func: row_number | rank | dense_rank | lag | lead | sum |
+    count | avg | min | max | first_value | last_value; args: child columns (none for COUNT(*) and the
+    ranking functions); partition: child columns; order: [(child column, ascending, nulls_first)];
+    frame: (ROWS | RANGE, lower, upper) with bounds (UNBOUNDED_PRECEDING | PRECEDING | CURRENT | FOLLOWING |
+    UNBOUNDED_FOLLOWING, offset); out: output column; params: (k, default) of lag / lead."""
+    func: str
+    args: tuple
+    partition: tuple
+    order: tuple
+    frame: tuple
+    out: str
+    params: tuple = ()
+
+
+class WindowSource(Source):
+    """Window functions over the child's rows: the child's columns followed by one column per call.
+    Calls with the same (partition, order) share one sort (executor.run_window)."""
+
+    def __init__(self, child: "LazyFrame", calls: Sequence[WindowCall]):
+        self.child, self.calls = child, list(calls)
+        self.schema = OrderedDict((n, child.col_type(n)) for n in child.columns)
+        for w in self.calls:
+            if w.func in ("row_number", "rank", "dense_rank", "count"):
+                self.schema[w.out] = (I64, "int64")
+            elif w.func == "avg":
+                self.schema[w.out] = (F64, "float64")
+            elif w.func == "sum":
+                dt = child.col_type(w.args[0])[0]
+                self.schema[w.out] = (F64, "float64") if dt == F64 else (I64, "int64")
+            else:
+                self.schema[w.out] = child.col_type(w.args[0])
 
 
 class LimitSource(Source):

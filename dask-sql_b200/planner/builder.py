@@ -65,6 +65,8 @@ class Binder:
             pred = self.bind_expr(q.where, plan.schema)
             if pred.contains_agg():
                 self.err("Aggregate functions are not allowed in WHERE")
+            if pred.contains_window():
+                self.err("Window functions are not allowed in WHERE")
             plan = P.Filter(plan, pred)
 
         # select list
@@ -80,6 +82,8 @@ class Binder:
                 items.append((self.bind_expr(e, plan.schema), alias))
         aliases = {a: e for e, a in items if a}
         having = self.bind_expr(q.having, plan.schema, aliases) if q.having is not None else None
+        if having is not None and having.contains_window():
+            self.err("Window functions are not allowed in HAVING")
         is_agg = bool(q.group_by) or any(e.contains_agg() for e, _ in items) or \
             (having is not None and having.contains_agg())
 
@@ -95,6 +99,8 @@ class Binder:
                     group_exprs.append(aliases[g.parts[0]])
                 else:
                     group_exprs.append(self.bind_expr(g, plan.schema))
+                if group_exprs[-1].contains_window():
+                    self.err("Window functions are not allowed in GROUP BY")
             agg_calls: List[PyExpr] = []
 
             def collect(e: PyExpr):
@@ -102,7 +108,7 @@ class Binder:
                     if not any(a.display() == e.display() for a in agg_calls):
                         agg_calls.append(e)
                     return
-                for c in e.args:
+                for c in e.args + e.window_exprs():
                     collect(c)
 
             for e, _ in items:
@@ -123,21 +129,24 @@ class Binder:
                              "aggregate function")
                 out = e.clone()
                 out.args = [rewrite(a) for a in e.args]
+                if e.window is not None:            # a window over the groups: its keys name group outputs
+                    out.window = e.window.map(rewrite)
                 return out
 
             plan = agg_plan
             if having is not None:
                 plan = P.Filter(plan, rewrite(having))
+            plan, exprs = self._windows(plan, [rewrite(e) for e, _ in items])
             proj = []
-            for e, alias in items:
-                r = rewrite(e)
+            for r, (e, alias) in zip(exprs, items):
                 name = alias if alias else None
                 if name is None and e.kind != "column":
                     name = None  # display name of the aggregate output column
                 proj.append(PyExpr("alias", r.sql_type, name=name, args=[r]) if name else r)
             plan = P.Projection(plan, proj)
         else:
-            proj = [PyExpr("alias", e.sql_type, name=a, args=[e]) if a else e for e, a in items]
+            plan, exprs = self._windows(plan, [e for e, _ in items])
+            proj = [PyExpr("alias", e.sql_type, name=a, args=[e]) if a else e for e, (_, a) in zip(exprs, items)]
             plan = P.Projection(plan, proj)
 
         if q.distinct:
@@ -150,6 +159,8 @@ class Binder:
                     b = P.col(f.qualifier, f.getName(), f.sql_type)
                 else:
                     b = self.bind_expr(e, plan.schema, order_by_fallback=items)
+                    if b.contains_window():
+                        self.err("ORDER BY refers to a window function by its alias only")
                 keys.append((b, asc, (not asc) if nulls_first is None else nulls_first))
             plan = P.Sort(plan, keys)
         if q.limit is not None or q.offset is not None:
@@ -157,6 +168,26 @@ class Binder:
             skip = q.offset.value if q.offset is not None else 0
             plan = P.Limit(plan, skip, fetch)
         return plan
+
+    def _windows(self, plan, exprs):
+        """Window calls of the select list become fields of one Window node on top of `plan` (the
+        input, or the aggregate and its HAVING filter); the select list then reads those fields."""
+        calls: List[PyExpr] = []
+
+        def lift(e: PyExpr) -> PyExpr:
+            if e.kind == "window":
+                d = e.display()
+                if not any(c.display() == d for c in calls):
+                    calls.append(e)
+                return P.col(None, d, e.sql_type)
+            if not e.contains_window():
+                return e
+            out = e.clone()
+            out.args = [lift(a) for a in e.args]
+            return out
+
+        exprs = [lift(e) for e in exprs]
+        return (P.Window(plan, calls) if calls else plan), exprs
 
     def _empty_relation(self):
         p = P.LogicalPlan()
@@ -291,6 +322,8 @@ class Binder:
             return PyExpr("case", ty, args=args)
         if k == "func":
             name = e.name
+            if e.over is not None:
+                return self.bind_window(e, rec)
             if name in P.AGG_FUNCS:
                 name = "AVG" if name == "MEAN" else name
                 args = [] if e.star else [rec(a) for a in e.args]
@@ -298,6 +331,8 @@ class Binder:
                     self.err(f"{name} takes exactly one argument")
                 if any(a.contains_agg() for a in args):
                     self.err("Aggregate function calls cannot be nested")
+                if any(a.contains_window() for a in args):
+                    self.err("Window function calls cannot be nested in an aggregate")
                 if name == "COUNT":
                     ty = "BIGINT"
                 elif name == "AVG" or name.startswith(("STDDEV", "VAR")):
@@ -313,3 +348,59 @@ class Binder:
                 return PyExpr("scalarfn", _norm_type(args[0].sql_type), name="abs", args=args)
             self.err(f"Function {name} is outside the int64/float64 hot path of the B200 layer")
         self.err(f"Unsupported expression {k}")
+
+    _FRAME_ORDER = {"UNBOUNDED_PRECEDING": 0, "PRECEDING": 1, "CURRENT": 2, "FOLLOWING": 3, "UNBOUNDED_FOLLOWING": 4}
+
+    def bind_window(self, e: Node, rec) -> PyExpr:
+        """f(args) OVER (...) -> PyExpr("window").  Output types: ROW_NUMBER / RANK / DENSE_RANK / COUNT
+        BIGINT, SUM int64 for integer and boolean input, AVG DOUBLE, the rest the argument's type."""
+        name = "AVG" if e.name == "MEAN" else e.name
+        if name not in P.WINDOW_FUNCS:
+            raise NotImplementedError(f"window function {name} is not supported")
+        if e.distinct:
+            raise NotImplementedError(f"{name}(DISTINCT ...) OVER (...) is not supported")
+        if e.filter is not None:
+            raise NotImplementedError(f"FILTER (WHERE ...) on the window function {name} is not supported")
+        if e.star and name != "COUNT":
+            self.err(f"{name}(*) is not a window function")
+        args = [] if e.star else [rec(a) for a in e.args]
+        spec = e.over
+        partition = [rec(p) for p in spec.partition]
+        order = [(rec(x), asc, (not asc) if nf is None else nf) for x, asc, nf in spec.order]
+        if any(x.contains_window() for x in args + partition + [o[0] for o in order]):
+            self.err("Window function calls cannot be nested")
+        nargs = {"ROW_NUMBER": (0, 0), "RANK": (0, 0), "DENSE_RANK": (0, 0), "LAG": (1, 3), "LEAD": (1, 3),
+                 "COUNT": (0, 1)}.get(name, (1, 1))
+        if not nargs[0] <= len(args) <= nargs[1]:
+            self.err(f"{name} takes {nargs[0]}..{nargs[1]} argument(s) in a window, got {len(args)}")
+        if name == "COUNT" and not args and not e.star:
+            self.err("COUNT() needs an argument or *")
+        if name in ("LAG", "LEAD"):
+            if len(args) > 1:
+                k = args[1]
+                if k.kind != "literal" or not isinstance(k.value, int) or isinstance(k.value, bool) or k.value < 0:
+                    self.err(f"the offset of {name} must be a non-negative integer literal")
+            if len(args) > 2 and args[2].kind != "literal":
+                self.err(f"the default of {name} must be a literal")
+        if name in ("ROW_NUMBER", "RANK", "DENSE_RANK", "COUNT"):
+            ty = "BIGINT"
+        elif name == "AVG":
+            ty = "DOUBLE"
+        elif name == "SUM":
+            ty = "BIGINT" if args[0].sql_type == "BOOLEAN" else _norm_type(args[0].sql_type)
+        else:
+            ty = args[0].sql_type
+        frame = spec.frame
+        if frame is not None:
+            unit, lo, hi = frame
+            for kind, off in (lo, hi):
+                if off is not None and (not isinstance(off, int) or off > (1 << 31) - 1):
+                    self.err(f"window frame offsets must be integers from 0 to 2^31-1, got {off}")
+            if unit == "RANGE" and any(b[0] in ("PRECEDING", "FOLLOWING") for b in (lo, hi)):
+                raise NotImplementedError("RANGE frames with a numeric offset are not supported "
+                                          "(use ROWS, or UNBOUNDED / CURRENT ROW bounds)")
+            if lo[0] == "UNBOUNDED_FOLLOWING" or hi[0] == "UNBOUNDED_PRECEDING" or \
+                    self._FRAME_ORDER[lo[0]] > self._FRAME_ORDER[hi[0]]:
+                self.err(f"invalid window frame: {unit} BETWEEN {lo[0]} AND {hi[0]}")
+        return PyExpr("window", ty, name=name, args=args, value="*" if e.star else None,
+                      window=P.WindowSpec(partition, order, frame))

@@ -151,6 +151,21 @@ def push_filters(plan: P.LogicalPlan, preds: List[PyExpr]) -> P.LogicalPlan:
         new = P.Aggregate(push_filters(child, down), plan.group_exprs, plan.agg_exprs)
         return _wrap(new, keep)
 
+    if isinstance(plan, P.Window):
+        # a filter decides which rows the windows see: only one over columns that every window
+        # partitions by removes whole partitions and may go below; filters on window outputs stay above
+        child = plan.inputs[0]
+        shared = None
+        for w in plan.window_exprs:
+            keys = {e.display() for e in w.window.partition if e.kind == "column"}
+            shared = keys if shared is None else shared & keys
+        down, keep = [], []
+        for p in preds:
+            cols = p.columns()
+            (down if cols and shared and all(c.display() in shared for c in cols) else keep).append(p)
+        new = P.Window(push_filters(child, down), plan.window_exprs)
+        return _wrap(new, keep)
+
     # Distinct / Sort / Limit / CrossJoin / Explain: optimise below, keep predicates above
     plan.inputs = [push_filters(i, []) for i in plan.inputs]
     return _wrap(plan, preds)
@@ -207,6 +222,8 @@ def _refresh_schemas(plan: P.LogicalPlan):
         plan.schema = list(l.schema) + ([] if plan.how in ("LEFTSEMI", "LEFTANTI") else list(r.schema))
     elif isinstance(plan, P.CrossJoin):
         plan.schema = list(plan.inputs[0].schema) + list(plan.inputs[1].schema)
+    elif isinstance(plan, P.Window):
+        plan.schema = plan._fields(plan.inputs[0].schema)
 
 
 def optimize(plan: P.LogicalPlan) -> P.LogicalPlan:

@@ -95,9 +95,79 @@ AGG_FUNCS = {"SUM", "AVG", "COUNT", "MIN", "MAX", "MEAN", "STDDEV", "STDDEV_SAMP
              "VAR_POP", "VARIANCE"}
 
 
+WINDOW_FUNCS = {"ROW_NUMBER", "RANK", "DENSE_RANK", "LAG", "LEAD", "SUM", "COUNT", "AVG", "MEAN", "MIN", "MAX",
+                "FIRST_VALUE", "LAST_VALUE", "SINGLE_VALUE"}
+_BOUND_TEXT = {"UNBOUNDED_PRECEDING": "UNBOUNDED PRECEDING", "CURRENT": "CURRENT ROW",
+               "UNBOUNDED_FOLLOWING": "UNBOUNDED FOLLOWING"}
+
+
+class WindowSpec:
+    """The OVER (...) of a window call: partition expressions, sort keys [(expr, asc, nulls_first)] and
+    the frame (unit, lower, upper) with bounds (kind, offset) -- None when the query gives none."""
+
+    def __init__(self, partition, order, frame):
+        self.partition, self.order, self.frame = list(partition), list(order), frame
+
+    def exprs(self):
+        return self.partition + [e for e, _, _ in self.order]
+
+    def map(self, fn) -> "WindowSpec":
+        return WindowSpec([fn(e) for e in self.partition], [(fn(e), a, nf) for e, a, nf in self.order], self.frame)
+
+    def display(self) -> str:
+        parts = []
+        if self.partition:
+            parts.append(f"PARTITION BY [{', '.join(e.display() for e in self.partition)}]")
+        if self.order:
+            keys = ", ".join(f"{e.display()} {'ASC' if a else 'DESC'} NULLS {'FIRST' if nf else 'LAST'}"
+                             for e, a, nf in self.order)
+            parts.append(f"ORDER BY [{keys}]")
+        if self.frame is not None:
+            unit, lo, hi = self.frame
+            show = lambda b: _BOUND_TEXT.get(b[0]) or f"{b[1]} {b[0]}"  # noqa: E731
+            parts.append(f"{unit} BETWEEN {show(lo)} AND {show(hi)}")
+        return " ".join(parts)
+
+
+class WindowFrame:
+    """getWindowFrame() of the Window node (the reference reads it at window.py:283-314)."""
+
+    def __init__(self, unit, lo, hi):
+        self.unit, self.lo, self.hi = unit, lo, hi
+
+    def getFrameUnits(self):
+        return self.unit
+
+    def getLowerBound(self):
+        return WindowFrameBound(*self.lo)
+
+    def getUpperBound(self):
+        return WindowFrameBound(*self.hi)
+
+
+class WindowFrameBound:
+    def __init__(self, kind, offset):
+        self.kind, self.offset = kind, offset
+
+    def isUnbounded(self):
+        return self.kind.startswith("UNBOUNDED")
+
+    def isPreceding(self):
+        return self.kind.endswith("PRECEDING")
+
+    def isFollowing(self):
+        return self.kind.endswith("FOLLOWING")
+
+    def isCurrentRow(self):
+        return self.kind == "CURRENT"
+
+    def getOffset(self):
+        return self.offset if self.kind in ("PRECEDING", "FOLLOWING") else None
+
+
 class PyExpr:
     """kind: column | literal | binary | not | isnull | isnotnull | negative | between | inlist |
-    cast | case | agg | alias | scalarfn | istrue"""
+    cast | case | agg | alias | scalarfn | istrue | window (name = function, args, window = WindowSpec)"""
 
     def __init__(self, kind, sql_type, **kw):
         self.kind = kind
@@ -110,6 +180,7 @@ class PyExpr:
         self.negated = kw.get("negated", False)
         self.distinct = kw.get("distinct", False)
         self.filter: Optional["PyExpr"] = kw.get("filter")
+        self.window: Optional[WindowSpec] = kw.get("window")
         self.inputs: List["LogicalPlan"] = []   # plans whose concatenated schema getIndex() indexes
 
     # -- construction helpers
@@ -119,10 +190,15 @@ class PyExpr:
             a.with_inputs(inputs)
         if self.filter is not None:
             self.filter.with_inputs(inputs)
+        for e in self.window_exprs():
+            e.with_inputs(inputs)
         return self
 
+    def window_exprs(self):
+        return self.window.exprs() if self.window is not None else []
+
     def children(self):
-        return self.args + ([self.filter] if self.filter is not None else [])
+        return self.args + ([self.filter] if self.filter is not None else []) + self.window_exprs()
 
     def columns(self, out=None):
         out = [] if out is None else out
@@ -133,12 +209,18 @@ class PyExpr:
         return out
 
     def contains_agg(self):
-        return self.kind == "agg" or any(c.contains_agg() for c in self.args)
+        """A group aggregate somewhere in the expression.  A window call is not one, but its arguments,
+        partition and sort keys may hold some: SUM(SUM(v)) OVER () runs after the GROUP BY."""
+        return self.kind == "agg" or any(c.contains_agg() for c in self.args + self.window_exprs())
+
+    def contains_window(self):
+        return self.kind == "window" or any(c.contains_window() for c in self.children())
 
     def clone(self):
         e = PyExpr(self.kind, self.sql_type, qualifier=self.qualifier, name=self.name, value=self.value,
                    op=self.op, args=[a.clone() for a in self.args], negated=self.negated,
-                   distinct=self.distinct, filter=self.filter.clone() if self.filter is not None else None)
+                   distinct=self.distinct, filter=self.filter.clone() if self.filter is not None else None,
+                   window=self.window.map(lambda x: x.clone()) if self.window is not None else None)
         e.inputs = self.inputs
         return e
 
@@ -197,6 +279,10 @@ class PyExpr:
             return self.args[0].display()
         if k == "scalarfn":
             return f"{self.name.lower()}({', '.join(a.display() for a in self.args)})"
+        if k == "window":
+            inner = "*" if self.value == "*" else ", ".join(a.display() for a in self.args)
+            spec = self.window.display()
+            return f"{self.name}({inner})" + (f" {spec}" if spec else "")
         return k
 
     __repr__ = display
@@ -223,7 +309,8 @@ class PyExpr:
         return {"column": "Column", "literal": "Literal", "alias": "Alias", "agg": "AggregateFunction",
                 "binary": "BinaryExpr", "not": "Not", "isnull": "IsNull", "isnotnull": "IsNotNull",
                 "negative": "Negative", "between": "Between", "inlist": "InList", "cast": "Cast",
-                "case": "Case", "scalarfn": "ScalarFunction", "istrue": "IsTrue"}[self.kind]
+                "case": "Case", "scalarfn": "ScalarFunction", "istrue": "IsTrue",
+                "window": "WindowFunction"}[self.kind]
 
     def column_name(self, rel=None) -> str:
         return self.display()
@@ -654,6 +741,56 @@ class Sort(LogicalPlan):
 
     def describe(self):
         return "Sort: " + ", ".join(f"{e.display()} {'ASC' if a else 'DESC'}" for e, a, _ in self.keys)
+
+
+class Window(LogicalPlan):
+    """Window functions over the input rows: the input's fields followed by one field per window call
+    (named by its display).  The method surface is the one DaskWindowPlugin calls
+    (dask_sql/physical/rel/logical/window.py:233-426): getGroups() lists the window calls, and the
+    other accessors take one of them."""
+    node_type = "Window"
+
+    def __init__(self, child, window_exprs: Sequence[PyExpr]):
+        super().__init__([child])
+        self.window_exprs = list(window_exprs)
+        self.schema = self._fields(child.schema)
+
+    def _fields(self, child_schema):
+        n = len(child_schema)
+        return list(child_schema) + [RelDataTypeField(None, e.display(), e.sql_type, n + i)
+                                     for i, e in enumerate(self.window_exprs)]
+
+    def window(self):
+        return self
+
+    def getGroups(self):
+        return list(self.window_exprs)
+
+    def getPartitionExprs(self, w: PyExpr):
+        return list(w.window.partition)
+
+    def getSortExprs(self, w: PyExpr):
+        out = []
+        for e, asc, nulls_first in w.window.order:
+            s = PyExpr("sort", e.sql_type, args=[e]).with_inputs(self.inputs)
+            s.ascending, s.nulls_first = asc, nulls_first
+            out.append(s)
+        return out
+
+    def getWindowFrame(self, w: PyExpr):
+        return WindowFrame(*w.window.frame) if w.window.frame is not None else None
+
+    def getWindowFuncName(self, w: PyExpr):
+        return w.name
+
+    def getArgs(self, w: PyExpr):
+        return list(w.args)
+
+    def expressions(self):
+        return list(self.window_exprs)
+
+    def describe(self):
+        return f"Window: windowExpr=[[{', '.join(e.display() for e in self.window_exprs)}]]"
 
 
 class Limit(LogicalPlan):

@@ -12,7 +12,15 @@ that crate cannot be built here (no rustc/cargo), so this is a small recursive-d
 
 Expressions: literals, [qualifier.]column, + - * / %, comparisons, AND OR NOT, IS [NOT] NULL,
 [NOT] BETWEEN, [NOT] IN (list), CAST(e AS type), CASE WHEN, function calls incl. aggregates with
-DISTINCT and FILTER (WHERE ...).
+DISTINCT and FILTER (WHERE ...), and window calls
+
+  f(args) OVER ([PARTITION BY e, ...] [ORDER BY e [ASC|DESC] [NULLS FIRST|LAST], ...]
+                [{ROWS | RANGE} {BETWEEN bound AND bound | bound}])
+  bound  := UNBOUNDED PRECEDING | n PRECEDING | CURRENT ROW | n FOLLOWING | UNBOUNDED FOLLOWING
+
+OVER / PARTITION / ROWS / RANGE / PRECEDING / FOLLOWING / UNBOUNDED / CURRENT / ROW are contextual
+words as well: OVER starts a window only directly after a call's ")" and before "(", so columns and
+aliases called over, rows, range or row keep parsing as before.
 
 Statements around the path (custom statements of the reference's parser, src/parser.rs):
   CREATE [OR REPLACE] TABLE|VIEW [IF NOT EXISTS] [schema.]name AS [(] query [)]
@@ -255,21 +263,7 @@ class Parser:
         order_by = []
         if self.eat_kw("ORDER"):
             self.expect_kw("BY")
-            while True:
-                e = self.parse_expr()
-                asc = True
-                if self.eat_kw("DESC"):
-                    asc = False
-                else:
-                    self.eat_kw("ASC")
-                nulls_first = None
-                if self.eat_kw("NULLS"):
-                    nulls_first = bool(self.eat_kw("FIRST"))
-                    if not nulls_first:
-                        self.expect_kw("LAST")
-                order_by.append((e, asc, nulls_first))
-                if not self.eat_op(","):
-                    break
+            order_by = self.parse_order_items()
         limit = offset = None
         if self.eat_kw("LIMIT"):
             limit = self.parse_expr()
@@ -277,6 +271,69 @@ class Parser:
             offset = self.parse_expr()
         return Node("select", distinct=distinct, items=items, source=source, where=where, group_by=group_by,
                     having=having, order_by=order_by, limit=limit, offset=offset, ctes=[])
+
+    def parse_order_items(self):
+        """e [ASC|DESC] [NULLS FIRST|LAST], ... -> [(e, asc, nulls_first or None)]"""
+        items = []
+        while True:
+            e = self.parse_expr()
+            asc = True
+            if self.eat_kw("DESC"):
+                asc = False
+            else:
+                self.eat_kw("ASC")
+            nulls_first = None
+            if self.eat_kw("NULLS"):
+                nulls_first = bool(self.eat_kw("FIRST"))
+                if not nulls_first:
+                    self.expect_kw("LAST")
+            items.append((e, asc, nulls_first))
+            if not self.eat_op(","):
+                return items
+
+    def parse_window_spec(self) -> Node:
+        """The parenthesised part after OVER (the opening "(" is consumed)."""
+        partition, order, frame = [], [], None
+        if self.eat_word("PARTITION"):
+            self.expect_kw("BY")
+            partition.append(self.parse_expr())
+            while self.eat_op(","):
+                partition.append(self.parse_expr())
+        if self.eat_kw("ORDER"):
+            self.expect_kw("BY")
+            order = self.parse_order_items()
+        unit = self.eat_word("ROWS", "RANGE")
+        if unit:
+            if self.eat_kw("BETWEEN"):
+                lo = self.parse_frame_bound()
+                self.expect_kw("AND")
+                hi = self.parse_frame_bound()
+            else:                               # "ROWS 3 PRECEDING" = BETWEEN 3 PRECEDING AND CURRENT ROW
+                lo, hi = self.parse_frame_bound(), ("CURRENT", 0)
+            frame = (unit, lo, hi)
+        self.expect_op(")")
+        return Node("window", partition=partition, order=order, frame=frame)
+
+    def parse_frame_bound(self):
+        """-> (kind, offset), kind in UNBOUNDED_PRECEDING | PRECEDING | CURRENT | FOLLOWING | UNBOUNDED_FOLLOWING"""
+        if self.eat_word("UNBOUNDED"):
+            d = self.eat_word("PRECEDING", "FOLLOWING")
+            if d is None:
+                self.error("Expected PRECEDING or FOLLOWING")
+            return ("UNBOUNDED_" + d, None)
+        if self.eat_word("CURRENT"):
+            self.expect_word("ROW")
+            return ("CURRENT", 0)
+        t = self.cur
+        if t.kind == "num":
+            self.i += 1
+            d = self.eat_word("PRECEDING", "FOLLOWING")
+            if d is None:
+                self.error("Expected PRECEDING or FOLLOWING")
+            if not re.fullmatch(r"\d+", t.val):
+                return (d, float(t.val))          # rejected by the binder with a clear message
+            return (d, int(t.val))
+        self.error("Expected a window frame bound")
 
     def parse_select_item(self):
         if self.eat_op("*"):
@@ -506,7 +563,11 @@ class Parser:
                     self.expect_kw("WHERE")
                     filt = self.parse_expr()
                     self.expect_op(")")
-                return Node("func", name=name.upper(), args=args, distinct=distinct, star=star, filter=filt)
+                over = None
+                if self.at_word("OVER") and self.toks[self.i + 1].kind == "op" and self.toks[self.i + 1].val == "(":
+                    self.i += 2
+                    over = self.parse_window_spec()
+                return Node("func", name=name.upper(), args=args, distinct=distinct, star=star, filter=filt, over=over)
             parts = [name]
             while self.eat_op("."):
                 parts.append(self.ident())

@@ -542,6 +542,82 @@ typedef struct b2_starlookup {
 int32_t b2_star_agg(const b2_scan_t* scan, int32_t fk_col, const b2_starlookup_t* lk,
                     const b2_agg_t* aggs, int32_t naggs, const b2_aggstate_t* st, void* stream);
 
+/* ---- window functions: f(...) OVER (PARTITION BY ... ORDER BY ... ROWS|RANGE ...) ---------------
+ * Replaces the reference's per-partition pandas pass of DaskWindowPlugin
+ * (dask_sql/physical/rel/logical/window.py:145-198, map_on_each_group: sort, then expanding() /
+ * rolling(Indexer) per group; and :330-332, groupby(partition keys).apply(...)).  All entry points
+ * work on columns already sorted by (partition keys, order keys) -- b2_iota + b2_sort_by per key,
+ * then b2_gather -- so a partition and a peer group (rows with equal ORDER BY values) are each a
+ * contiguous row range.  Row ranges are int32: the input holds < 2^31 rows. */
+#define B2_WIN_MAX_KEYS 8
+
+/* per-row segment arrays (int32[n] each, caller-allocated): [part_start, part_end) is the row's
+ * partition, [peer_start, peer_end) its peer group, dense[i] the number of peer-group starts in
+ * rows 0..i (DENSE_RANK helper). */
+typedef struct b2_wsegs {
+  int32_t* part_start;
+  int32_t* part_end;
+  int32_t* peer_start;
+  int32_t* peer_end;
+  int32_t* dense;
+} b2_wsegs_t;
+
+/* window frame.  kind B2_WB_UNBOUNDED: UNBOUNDED PRECEDING (lower bound) / UNBOUNDED FOLLOWING
+ * (upper bound).  kind B2_WB_OFFSET: a row offset from the current row, -a = a PRECEDING,
+ * 0 = CURRENT ROW, +b = b FOLLOWING.  range != 0: RANGE frame, whose B2_WB_OFFSET bounds must be 0
+ * and mean the first / last peer of the current row. */
+#define B2_WB_UNBOUNDED 0
+#define B2_WB_OFFSET    1
+typedef struct b2_wframe {
+  int32_t range;
+  int32_t lo_kind;
+  int32_t hi_kind;
+  int32_t pad_;
+  int64_t lo;
+  int64_t hi;
+} b2_wframe_t;
+
+/* window functions (b2_window_rank / b2_window_agg op) */
+#define B2_WIN_ROW_NUMBER  0
+#define B2_WIN_RANK        1
+#define B2_WIN_DENSE_RANK  2
+#define B2_WIN_SUM         3   /* int64 (wrapping) for B2_I64 input, float64 for B2_F64 */
+#define B2_WIN_COUNT       4   /* non-NULL values; val->data == NULL: COUNT(*) */
+#define B2_WIN_AVG         5   /* float64 */
+#define B2_WIN_MIN         6
+#define B2_WIN_MAX         7
+#define B2_WIN_FIRST       8   /* value at the frame's first row (NULL if that value is NULL) */
+#define B2_WIN_LAST        9
+
+/* device scratch of b2_window_segments / b2_window_agg for n rows */
+int64_t b2_window_ws_bytes(int64_t n);
+
+/* keys[0..npart) = partition keys, keys[npart..nkeys) = order keys, all gathered into sorted order.
+ * NULL equals NULL, NaN is NULL, -0.0 equals 0.0 (the conventions of b2_sort_by's key image).
+ * Starts: one pass with a decoupled look-back of the tile carries; ends: scattered at each
+ * segment's last row and gathered.  Every array of `segs` is written. */
+int32_t b2_window_segments(const b2_col_t* keys, int32_t npart, int32_t nkeys, int64_t n, const b2_wsegs_t* segs,
+                           void* ws, void* stream);
+
+/* ROW_NUMBER / RANK / DENSE_RANK -> int64[n] (window.py:187-190 computes ROW_NUMBER as range(1, len+1)) */
+int32_t b2_window_rank(int32_t op, int64_t n, const b2_wsegs_t* segs, int64_t* out, void* stream);
+
+/* LAG (offset = -k) / LEAD (offset = +k): out[i] = val[i + offset] when that row is in i's partition,
+ * else the default (has_default: default_raw, the value's 64-bit pattern; else NULL).  val: B2_I64 or
+ * B2_F64; out has val's type; out_valid: (n+31)/32 words. */
+int32_t b2_window_offset(const b2_col_t* val, int64_t n, int64_t offset, int32_t has_default, int64_t default_raw,
+                         const b2_wsegs_t* segs, void* out, uint32_t* out_valid, void* stream);
+
+/* Framed aggregate (window.py:161-192: expanding() / rolling() per group).  val: B2_I64 or B2_F64.
+ * Lower bound UNBOUNDED: segmented inclusive scan read at the frame end; upper bound UNBOUNDED: reverse
+ * scan read at the frame start; both bounded: evaluated over the frame (int64 SUM / COUNT over frames
+ * wider than 32 rows: difference of the exact wrapping prefix sums).  Float scans combine tile carries
+ * in a fixed order, so results are bit-identical from run to run.  Empty frame or no non-NULL value:
+ * NULL (COUNT: 0).  out: int64 (COUNT, int SUM/MIN/MAX/FIRST/LAST) or float64 (AVG, float input);
+ * out_valid: (n+31)/32 words or NULL for COUNT.  ws >= b2_window_ws_bytes(n). */
+int32_t b2_window_agg(const b2_col_t* val, int32_t op, const b2_wframe_t* frame, int64_t n, const b2_wsegs_t* segs,
+                      void* out, uint32_t* out_valid, void* ws, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
